@@ -20,6 +20,13 @@ argmin selected. The default workload is BASELINE.json configs[2] ("crowd stress
 `--impl reference` times the reference's CPU implementation of the path (oracle/_ref: its own sources compiled in
 place; falls back to the oracle restatement if that library is absent), FP64, all host threads, on a bounded candidate
 sample of the same workload.
+
+`--steps K` is the number of timed steps of the workload (default 40; cfg4: replay cycles, default 1000).
+`--dump-outputs DIR` writes, after the timed steps, what the timed path returned in its last step as DIR/<name>.npy
+(float64): every field of the HmpResult records (result_<field>, leading axis = scene; timings left out) and the
+per-candidate totals (explored_totals, or a fixed seeded sample of them with its flat indices where they exceed 2^20).
+The inputs are seeded, so two builds run with the same arguments can be compared output for output. In a multi-GPU run
+of the batched workload (cfg3) the file holds rank 0's share of the worlds (s mod N == 0, in that order).
 """
 from __future__ import annotations
 
@@ -39,6 +46,38 @@ import numpy as np  # noqa: E402
 
 METRIC = "candidate trajectories scored/sec"
 UNIT = "candidates/s"
+
+
+DUMP_MAX_BYTES = 64 << 20
+DUMP_MAX_TOTALS = 1 << 20
+
+
+def _result_arrays(results) -> dict:
+    """HmpResult records -> one float64 array per field (leading axis = scene); timings and padding are left out."""
+    from humap_local_planner_b200 import capi
+    out = {}
+    for name, _ in capi.HmpResult._fields_:
+        if name not in ("gpu_ms", "gpu_ms_select", "_pad"):
+            out["result_" + name] = np.array([np.array(getattr(r, name), dtype=np.float64) for r in results])
+    return out
+
+
+def _totals_arrays(totals: np.ndarray) -> dict:
+    """Per-candidate totals, or a fixed seeded sample of them (and its flat indices) where there are more than DUMP_MAX_TOTALS."""
+    if totals.size <= DUMP_MAX_TOTALS:
+        return {"explored_totals": totals}
+    idx = np.sort(np.random.default_rng(0).choice(totals.size, DUMP_MAX_TOTALS, replace=False))
+    return {"explored_totals_sample": totals[idx], "explored_totals_sample_index": idx.astype(np.float64)}
+
+
+def _write_outputs(path: str, arrays: dict):
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def algorithmic_flops_per_candidate(cfg, params, n_static, n_dynamic, fis_on, T, K=8, V=16, c_cells=45):
@@ -180,10 +219,11 @@ def _make_scene_job(a):
                 local_goal=[bool(lg) for _, lg in sc.plans], hv=sc.hv_prev)
 
 
-def run_batched(args, rank, local_rank, world, barrier, steps, warmup, n_scenes):
+def run_batched(args, rank, local_rank, world, barrier, steps, warmup, n_scenes, dump=None):
     """BASELINE config 4: n_scenes independent worlds (seed = world index) x cfg3's 4096 candidates each, scene s -> rank
     s mod N, one hmp_plan_batch launch per rank per step, host gather of the per-scene argmins (no collective on the data
-    path). Total work is fixed, so this is STRONG scaling. Returns the JSON line (rank 0) or None.
+    path). Total work is fixed, so this is STRONG scaling. Returns the JSON line (rank 0) or None. A dict passed as `dump`
+    receives the outputs of this rank's last timed step.
 
       value  resident: costmaps, MapGrids and worlds already in HBM, hmp_replan_resident, CUDA events
       e2e    host buffers through the C ABI every step: hmp_compute_mapgrid_batch (uploads the costmaps -- 1 byte per cell --
@@ -259,10 +299,14 @@ def run_batched(args, rank, local_rank, world, barrier, steps, warmup, n_scenes)
     dev_ms = []
     for _ in range(steps):
         torch.cuda.synchronize()
-        dev_ms.append(pl.replan_resident()[0].gpu_ms)   # per-step inputs (n_local x 680 kB) exceed the 126 MB L2
+        last = pl.replan_resident()
+        dev_ms.append(last[0].gpu_ms)   # per-step inputs (n_local x 680 kB) exceed the 126 MB L2
     barrier()
     launches = pl.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if dump is not None:
+        dump.update(_result_arrays(last))
+        dump.update(_totals_arrays(pl.explored_totals(n_local * C)))
     t_dev = torch.tensor([sum(dev_ms) * 1e-3], dtype=torch.float64, device="cuda")
     e2e_t = []
     n_e2e = max(1, min(steps, 5))
@@ -360,7 +404,7 @@ def _ncu_counts():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=40)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 40; cfg4: replay cycles, default 1000)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--cfg", default=None, help="workload: cfg2 (default at 1 GPU: BASELINE config 3, the headline), cfg1, cfg0, "
@@ -374,6 +418,9 @@ def main():
     ap.add_argument("--no-config4", action="store_true", help="1 GPU: skip the nested config-4 (batched scenes) measurement")
     ap.add_argument("--precise", type=int, default=2, help="hmp_set_precision mode: 0 FP32 object loops, 1 FP64 (exact-parity mode), 2 FP32 sweep + FP64 refinement of the leaders")
     ap.add_argument("--layout", type=int, default=0, help="hmp_set_sweep_layout: 0 automatic, 1 one warp per candidate, 2 one thread per candidate")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step to DIR/<name>.npy (float64, at most 64 MB); "
+                         "cfg3 on N > 1 GPUs: rank 0's share of the worlds")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -384,6 +431,13 @@ def main():
         # 1 GPU: the configuration the metric is quoted on (64k candidates, one planning cycle = one GPU by design);
         # N > 1: the only configuration that shards (independent worlds), BASELINE config 4
         args.cfg = "cfg2" if world == 1 else "cfg3"
+    if args.steps is None:
+        args.steps = 1000 if args.cfg == "cfg4" else 40
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    dump = {} if args.dump_outputs else None
 
     if args.impl == "reference":
         run_reference(args, rank, world)
@@ -405,16 +459,22 @@ def main():
 
     if args.cfg == "cfg4":
         from humap_local_planner_b200 import replay
-        line = replay.bench_line(args, rank, local_rank, world, barrier) if hasattr(replay, "bench_line") else None
+        line = replay.bench_line(args, rank, local_rank, world, barrier, dump=dump)
         if rank == 0 and line is not None:
+            if dump is not None:
+                last = dump.pop("replay_last_result")
+                dump.update(_result_arrays([] if last is None else [last]))
+                _write_outputs(args.dump_outputs, dump)
             print(json.dumps(line))
         if world > 1:
             dist.destroy_process_group()
         return
 
     if args.cfg == "cfg3":
-        line = run_batched(args, rank, local_rank, world, barrier, args.steps, args.warmup, args.scenes)
+        line = run_batched(args, rank, local_rank, world, barrier, args.steps, args.warmup, args.scenes, dump=dump)
         if rank == 0:
+            if dump is not None:
+                _write_outputs(args.dump_outputs, dump)
             print(json.dumps(line))
         if world > 1:
             dist.destroy_process_group()
@@ -490,6 +550,10 @@ def main():
         barrier()
         wall_resident += time.perf_counter() - t_w0
         launches += pl.launch_count() - l0
+        if dump is not None and seed == n_seeds - 1:
+            # read before the e2e cycles below plan again
+            dump.update(_result_arrays([r]))
+            dump.update(_totals_arrays(pl.explored_totals(C)))
         # ---- e2e: host buffers through the public C-ABI, every step uploads the cycle's inputs and reads the result ----
         full_cycle()
         barrier()
@@ -702,6 +766,8 @@ def main():
         except Exception as e:   # the headline line must not depend on it
             line["config4"] = {"error": repr(e)}
     if rank == 0:
+        if dump is not None:
+            _write_outputs(args.dump_outputs, dump)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -4,7 +4,7 @@
  * signatures of humap_local_planner::SocialTrajectoryGenerator, so that HumapPlanner's call sites compile unchanged.
  *
  * Header-only; needs the reference's headers on the include path (include/humap_local_planner/...). It is NOT part of
- * libhmp_planner.so and uses no CUDA header. Compiled and tested here against /root/reference/include + the stand-in
+ * libhmp_planner.so and uses no CUDA header. Compiled and tested against $HMP_REFERENCE_DIR/include + the stand-in
  * third-party headers of oracle/ref_shim (tests/from_reference_test.cpp, tests/test_from_reference.py).
  *
  *   toHmpSampling(TrajectorySamplingParams)            humap_config.h:176-224 -> HmpSampling

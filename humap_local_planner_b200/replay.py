@@ -20,7 +20,7 @@ from typing import List, Optional
 import numpy as np
 
 from . import config, scenes
-from .capi import HmpObstacle, HmpPerson, HmpWorld, Planner
+from .capi import HmpObstacle, HmpPerson, HmpResult, HmpWorld, Planner
 
 XY_TOL, YAW_TOL = 0.1, 0.2     # src/humap_config_ros.cpp:63-64
 
@@ -37,6 +37,7 @@ class ReplayLog:
     escalated: int = 0                                        # plans redone as an exact FP64 sweep (hmp_set_escalation)
     parity_checked: int = 0
     parity_mismatch: int = 0
+    last_result: Optional[HmpResult] = None                   # HmpResult of the last MOVE cycle
 
 
 def _wrap(a):
@@ -144,6 +145,7 @@ def run_replay(planner: Planner, n_cycles: int = 1000, period: float = 0.05, see
             log.plan_ms.append(1e3 * (time.perf_counter() - t0))
             log.gpu_ms.append(res.gpu_ms)
             log.best.append(res.best_index)
+            log.last_result = res
             if hasattr(planner, "last_escalated") and planner.last_escalated() == 1:
                 log.escalated += 1
             if res.status == 0:
@@ -198,12 +200,13 @@ def summarize(log: ReplayLog) -> dict:
             "recoveries": log.recoveries}
 
 
-def bench_line(args, rank, local_rank, world, barrier) -> Optional[dict]:
+def bench_line(args, rank, local_rank, world, barrier, dump: Optional[dict] = None) -> Optional[dict]:
     """`bench.py --cfg cfg4`: BASELINE config 5 -- consecutive 20 Hz planning cycles with moving people and the
     init -> move -> adjust -> stop sequence; p50 / p99 latency of the full C-ABI cycle (costmap upload, four device wave
     fronts, footprint, plan in the configured precision mode, result read back) for the stock sampling (72 candidates) and
-    for the 64k-candidate grid. --steps = cycles per run (default 40 -> 1000). One process per GPU runs the same replay."""
-    cycles = 1000 if args.steps == 40 else max(50, args.steps)
+    for the 64k-candidate grid. --steps = cycles per run. One process per GPU runs the same replay. A dict passed as
+    `dump` receives the 64k replay's outputs: the last plan's HmpResult, the winner of every MOVE cycle, the robot poses."""
+    cycles = args.steps
     pl = Planner(local_rank)
     pl.set_precision(int(args.precise))
     pl.set_sweep_layout(int(args.layout))
@@ -211,8 +214,13 @@ def bench_line(args, rank, local_rank, world, barrier) -> Optional[dict]:
     barrier()
     l0 = pl.launch_count()
     small = summarize(run_replay(pl, cycles))
-    big = summarize(run_replay(pl, cycles, sampling_axes=config.SAMPLING_64K))
+    big_log = run_replay(pl, cycles, sampling_axes=config.SAMPLING_64K)
+    big = summarize(big_log)
     launches = pl.launch_count() - l0
+    if dump is not None:
+        dump["replay_last_result"] = big_log.last_result
+        dump["replay_best_index"] = np.array(big_log.best, dtype=np.float64)
+        dump["replay_robot_poses"] = np.array(big_log.poses, dtype=np.float64).reshape(-1, 3)
     barrier()
     pl.close()
     if rank != 0:

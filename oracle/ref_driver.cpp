@@ -1,6 +1,6 @@
 /*
  * ref_driver.cpp -- TEST INFRASTRUCTURE. Drives the reference's OWN first-party sources (compiled where they lie under
- * /root/reference by oracle/Makefile, target _ref/libhmp_ref.so, against the stand-in third-party headers of
+ * $HMP_REFERENCE_DIR by oracle/Makefile, target _ref/libhmp_ref.so, against the stand-in third-party headers of
  * oracle/ref_shim/) through the same flat inputs as the oracle's orc_plan, so that tests can compare
  *     reference sources  <->  oracle restatement (hmp_oracle.cpp)  <->  CUDA path
  * on identical scenes. Nothing under humap_local_planner_b200/ may include, link or load this.

@@ -14,6 +14,9 @@ from humap_local_planner_b200.capi import (HmpParams, HmpWorld, HmpSampling, Hmp
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 _LIB = os.path.join(ROOT, "oracle", "_build", "libhmp_oracle.so")
 _REF_LIB = os.path.join(ROOT, "oracle", "_ref", "libhmp_ref.so")
+# Optional checkout of the original humap_local_planner: the live comparisons compile its own sources where they lie
+# (oracle/Makefile and tests/Makefile read the same variable). Without it they skip.
+REFERENCE_DIR = os.environ.get("HMP_REFERENCE_DIR", "")
 _d, _i = C.c_double, C.c_int32
 _lib = None
 _ref_lib = None
@@ -65,17 +68,22 @@ def lib() -> C.CDLL:
     return _lib
 
 
+def reference_has(sub: str) -> bool:
+    """True when HMP_REFERENCE_DIR names a checkout of the original project that has `sub` (src, include)."""
+    return bool(REFERENCE_DIR) and os.path.isdir(os.path.join(REFERENCE_DIR, sub))
+
+
 def ref_available() -> bool:
     """True when oracle/_ref/libhmp_ref.so (the reference's own sources compiled against oracle/ref_shim) exists or can
-    be built here (needs /root/reference; on the GPU box only the prebuilt library is used)."""
-    return os.path.exists(_REF_LIB) or os.path.isdir("/root/reference/src")
+    be built from the checkout HMP_REFERENCE_DIR names."""
+    return os.path.exists(_REF_LIB) or reference_has("src")
 
 
 def ref_lib() -> C.CDLL:
     global _ref_lib
     if _ref_lib is None:
         lib()  # libhmp_oracle.so first: the stand-ins' orc_tp_* hooks resolve against it
-        if os.path.isdir("/root/reference/src"):   # incremental; on the GPU box the prebuilt library is used as is
+        if reference_has("src"):   # incremental; without the checkout a prebuilt library is used as is
             subprocess.run(["make", "-s", "-j8", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True)
         _ref_lib = C.CDLL(_REF_LIB)
         _ref_lib.ref_plan.argtypes = [C.POINTER(OrcPlanInput), C.POINTER(OrcPlanOutput)]

@@ -19,14 +19,14 @@ LIB = os.path.join(ROOT, "tests", "_build", "libfrom_reference_test.so")
 
 
 def _lib():
-    if os.path.isdir("/root/reference/include"):
-        import oracle_binding as ob
+    import oracle_binding as ob
+    if ob.reference_has("include"):
         ob.ref_lib()   # oracle/_ref/libhmp_ref.so
         from humap_local_planner_b200 import build as b
         b.build_library()
         subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "tests")], check=True)
     if not os.path.exists(LIB):
-        pytest.skip("tests/_build/libfrom_reference_test.so needs /root/reference to be built")
+        pytest.skip("tests/_build/libfrom_reference_test.so is built from the original project's headers (HMP_REFERENCE_DIR)")
     return C.CDLL(LIB)
 
 

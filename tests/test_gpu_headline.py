@@ -22,7 +22,7 @@ GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 def _full(name, seed):
     path = os.path.join(GOLD, f"ref_full_{name}_s{seed}.npz")
     if not os.path.exists(path):
-        pytest.skip(f"{os.path.basename(path)} missing: run tools/make_ref_golden_full.py where /root/reference exists")
+        pytest.skip(f"{os.path.basename(path)} missing: run tools/make_ref_golden_full.py with HMP_REFERENCE_DIR set")
     return np.load(path)
 
 

@@ -1,6 +1,6 @@
 """Pins the CPU oracle against the known-answer tests of the reference's own test suite.
 
-Every case below is transcribed from /root/reference/test/*.cpp (file:line cited per test); the
+Every case below is transcribed from the reference's test/*.cpp (file:line cited per test); the
 numbers are the reference's golden values (most of them produced by the author's MATLAB prototypes in
 scripts/). These tests run on CPU (`-m "not gpu"`).
 """

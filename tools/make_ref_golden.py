@@ -2,16 +2,21 @@
 """Generates tests/golden/ref_*.npz from the REFERENCE'S OWN sources.
 
 oracle/_ref/libhmp_ref.so is the reference's first-party code for the path (generator, SFM, World, FIS, conductor, the
-eleven first-party critics) compiled where it lies under /root/reference against the stand-in third-party headers of
-oracle/ref_shim/ (oracle/Makefile, target `ref`; driver oracle/ref_driver.cpp). /root/reference does not exist on the
-GPU box, so its outputs on the seeded synthetic scenes of humap_local_planner_b200/scenes.py are frozen here as small
-fixtures; tests/test_ref_golden.py (CPU: oracle vs fixtures) and tests/test_gpu_parity.py (GPU: CUDA path vs fixtures)
+eleven first-party critics) compiled where it lies in the checkout HMP_REFERENCE_DIR names, against the stand-in
+third-party headers of oracle/ref_shim/ (oracle/Makefile, target `ref`; driver oracle/ref_driver.cpp). Its outputs on the
+seeded synthetic scenes of humap_local_planner_b200/scenes.py are frozen as small fixtures so that the tests need no
+checkout; tests/test_ref_golden.py (CPU: oracle vs fixtures) and tests/test_gpu_parity.py (GPU: CUDA path vs fixtures)
 read them. Re-run after changing scenes.py / config.py defaults:
 
-    python tools/make_ref_golden.py
+    HMP_REFERENCE_DIR=<checkout> python tools/make_ref_golden.py          # tests/golden/ref_cycle_*.npz, ref_fis.npz
+    HMP_REFERENCE_DIR=<checkout> python tools/make_ref_golden.py --live   # tests/golden/ref_live_*.npz
+
+--live runs the comparisons of tests/test_ref_golden.py that have no fixture of their own with HMP_WRITE_REF_GOLDEN=1:
+each stores the compiled reference's outputs for its case, which the test reads where oracle/_ref is absent.
 """
 import hashlib
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -64,5 +69,13 @@ def main():
     print(path, os.path.getsize(path), "bytes; fired", int(out3[:, 2].sum()), "of", FIS_N)
 
 
+def main_live():
+    if not ob.ref_available():
+        sys.exit("oracle/_ref is not built and HMP_REFERENCE_DIR names no checkout of the reference")
+    env = dict(os.environ, HMP_WRITE_REF_GOLDEN="1")
+    subprocess.run([sys.executable, "-m", "pytest", "-q", os.path.join(ROOT, "tests", "test_ref_golden.py"), "-k", "compiled_reference"],
+                   check=True, env=env)
+
+
 if __name__ == "__main__":
-    main()
+    main_live() if "--live" in sys.argv[1:] else main()

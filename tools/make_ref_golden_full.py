@@ -6,8 +6,8 @@
 oracle/_ref/libhmp_ref.so (the reference's own sources compiled in place, oracle/Makefile target `ref`) scores EVERY
 candidate of the sampling grid without the early exit of SimpleScoredSamplingPlanner (full sums, so that the fixture also
 ranks the losers); the winner (first strict minimum = the reference's rule, humap_planner.cpp:1367) is then evaluated
-once more alone for its record (raw critics, seed twist, poses). /root/reference does not exist on the GPU box, hence the
-fixtures: tests/golden/ref_full_<cfg>_s<seed>.npz (cfg2: 65 536 totals, ~3.6 min on 16 threads each) and
+once more alone for its record (raw critics, seed twist, poses). Needs HMP_REFERENCE_DIR (a checkout of the reference); the
+fixtures let the tests run without one: tests/golden/ref_full_<cfg>_s<seed>.npz (cfg2: 65 536 totals, ~3.6 min on 16 threads each) and
 tests/golden/ref_full_cfg3_s0-7.npz (8 worlds x 4096). One process per candidate chunk (the stand-in MapGrid fill hook is a
 process-wide pointer, so threads are avoided here).
 """
