@@ -104,6 +104,11 @@ class HmpSample(C.Structure):
     _fields_ = [("amp", _d * NUM_AMPLIFIERS)]
 
 
+class HmpSceneCosts(C.Structure):
+    """Per-world scales and MapGrid shifts of a batch (hmp_set_scene_costs); same meaning as the fields of HmpCosts."""
+    _fields_ = [("scale", _d * NUM_COSTS), ("xshift", _d * NUM_MAPGRIDS), ("yshift", _d * NUM_MAPGRIDS)]
+
+
 class HmpResult(C.Structure):
     _fields_ = [
         ("status", _i), ("best_index", _i), ("n_candidates", _i), ("n_generated", _i), ("n_valid", _i), ("n_poses", _i),
@@ -151,7 +156,7 @@ ABI_SYMBOLS = (
     "hmp_set_sweep_layout", "hmp_last_sweep_mode", "hmp_last_num_leaders_round2",
     "hmp_compute_mapgrid_batch", "hmp_set_mapgrids_batch_f32", "hmp_last_num_scenes", "hmp_last_fallback_rounds",
     "hmp_debug_sweep_candidate", "hmp_host_alloc", "hmp_host_free",
-    "hmp_set_escalation", "hmp_last_unreliable_leaders", "hmp_last_escalated",
+    "hmp_set_escalation", "hmp_last_unreliable_leaders", "hmp_last_escalated", "hmp_set_scene_costs",
 )
 
 _LIB_PATH = os.environ.get("HMP_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libhmp_planner.so")
@@ -194,6 +199,8 @@ def load_library() -> C.CDLL:
     lib.hmp_set_mapgrids_batch_f32.restype = C.c_int
     lib.hmp_set_escalation.argtypes = [C.c_void_p, _i]
     lib.hmp_set_escalation.restype = C.c_int
+    lib.hmp_set_scene_costs.argtypes = [C.c_void_p, C.c_void_p, _i]
+    lib.hmp_set_scene_costs.restype = C.c_int
     for name in ("hmp_last_num_scenes", "hmp_last_fallback_rounds", "hmp_last_num_leaders_round2", "hmp_last_unreliable_leaders",
                  "hmp_last_escalated"):
         getattr(lib, name).argtypes = [C.c_void_p]
@@ -464,11 +471,23 @@ class Planner:
                                        _ptr(poses), MAX_STEPS if want_poses else 0))
         return res, (poses[: max(res.n_poses, 0)] if want_poses else None)
 
+    def set_scene_costs(self, costs):
+        """Per-world scales / MapGrid shifts of the following plan_batch calls: a sequence (or ctypes array) of HmpSceneCosts,
+        entry s for scene s. None or an empty sequence clears the table: every world uses the scales / shifts of set_params."""
+        n = 0 if costs is None else len(costs)
+        arr = None
+        if n:
+            arr = costs if isinstance(costs, C.Array) else (HmpSceneCosts * n)(*costs)
+        self._check(self._lib.hmp_set_scene_costs(self._ctx, arr, n))
+
     def plan_batch(self, worlds, cells: Optional[np.ndarray], grids: Optional[Sequence[np.ndarray]],
-                   sampling: HmpSampling, hv_prev: Optional[np.ndarray] = None):
+                   sampling: HmpSampling, hv_prev: Optional[np.ndarray] = None, scene_costs=None):
         """worlds: sequence of HmpWorld or a ctypes HmpWorld array; cells: [n][size_y][size_x] uint8 or None (costmaps of an
         earlier batch call stay); grids: 4 arrays [n][size_y][size_x] float64, or None (grids left resident by
-        compute_mapgrid_batch / set_mapgrids_batch_f32 / an earlier batch)."""
+        compute_mapgrid_batch / set_mapgrids_batch_f32 / an earlier batch). scene_costs: if given, set_scene_costs(scene_costs)
+        first; the table then stays for later batches until it is set again or cleared."""
+        if scene_costs is not None:
+            self.set_scene_costs(scene_costs)
         n = len(worlds)
         arr = worlds if isinstance(worlds, C.Array) else (HmpWorld * n)(*worlds)
         cells = None if cells is None else np.ascontiguousarray(cells, dtype=np.uint8)

@@ -9,7 +9,7 @@ from __future__ import annotations
 
 import math
 
-from .capi import (HmpParams, HmpSampling, NUM_AMPLIFIERS, NUM_MAPGRIDS)
+from .capi import (COST_NAMES, HmpParams, HmpSampling, HmpSceneCosts, NUM_AMPLIFIERS, NUM_COSTS, NUM_MAPGRIDS)
 
 ROBOT_INSCRIBED_RADIUS = 0.275
 PERSON_MODEL_RADIUS = 0.4
@@ -66,6 +66,46 @@ def default_params(resolution: float = 0.05, sim_time: float = 3.5, sim_granular
     c.unsat_whole_horizon, c.hd_whole_horizon, c.psi_whole_horizon = 0, 1, 1
     c.fsi_whole_horizon, c.ps_whole_horizon = 1, 1
     return p
+
+
+_ALIGNMENT, _UNSATURATED, _FFORMATION = (COST_NAMES.index(n) for n in ("alignment", "unsaturated", "fformation"))
+_GRID_ALIGNMENT, _GRID_GOAL_FRONT = 2, 3   # HmpMapGridIndex
+
+
+def local_scene_costs(params: HmpParams, world, people_xy=None, goal_within_group: bool = False, dist_to_group_edge: float = 0.0,
+                      inscribed_radius: float = ROBOT_INSCRIBED_RADIUS,
+                      person_model_radius: float = PERSON_MODEL_RADIUS) -> HmpSceneCosts:
+    """The per-cycle setScale / setXShift calls of HumapPlanner::updateLocalCosts (src/humap_planner.cpp:1054-1141) for one
+    robot, restated from adapter/from_reference.h (applyLocalCosts + minGapHumanRobot); one entry of Planner.set_scene_costs.
+
+    `params` holds the base values, as toHmpParams / default_params leave them: scale[] (MapGrid scales x resolution) and
+    forward_point_distance as the xshift of the goal-front grid. `world` gives pose_ and goal_; people_xy: [n][2] positions of
+    the people of people_env_model_ (None: no people). GroupIntrusionDetector is not restated: whether the goal lies inside an
+    F-formation and its distance to that group's edge are inputs."""
+    c = params.costs
+    out = HmpSceneCosts()
+    for k in range(NUM_COSTS):
+        out.scale[k] = c.scale[k]
+    for g in range(NUM_MAPGRIDS):
+        out.xshift[g], out.yshift[g] = c.xshift[g], c.yshift[g]
+    forward_point_distance = c.xshift[_GRID_GOAL_FRONT]
+    min_gap = float("inf")   # std::numeric_limits<double>::max() without people, :1068-1083
+    for px, py in ([] if people_xy is None else people_xy):
+        gap = math.hypot(px - world.robot_x, py - world.robot_y) - person_model_radius - inscribed_radius
+        min_gap = min(max(0.0, gap), min_gap)
+    fwd = min(min_gap, forward_point_distance)                                   # :1085
+    out.xshift[_GRID_GOAL_FRONT] = fwd                                           # :1104
+    out.xshift[_GRID_ALIGNMENT] = fwd                                            # :1112
+    dist_to_goal = math.hypot(world.goal_x - world.robot_x, world.goal_y - world.robot_y)   # :1056
+    out.scale[_ALIGNMENT] = 0.0 if dist_to_goal <= forward_point_distance else c.scale[_ALIGNMENT]   # :1107-1111
+    if goal_within_group:                                                        # :1116-1127
+        dist_to_group = max(dist_to_group_edge - inscribed_radius, 0.0)
+        out.scale[_FFORMATION] = (1.0 - math.exp(-0.7 * dist_to_group)) * c.scale[_FFORMATION]
+    threshold = 3.0 * inscribed_radius                                           # :1130-1140
+    if dist_to_goal <= threshold:
+        lin_val = c.scale[_UNSATURATED] / threshold * dist_to_goal
+        out.scale[_UNSATURATED] = min(max(lin_val, 0.0), c.scale[_UNSATURATED])
+    return out
 
 
 def amplifier_samples(amp_min: float, amp_max: float, granularity: float):

@@ -204,6 +204,7 @@ struct HmpContext {
 	int refine_min_leaders = 16;     // the best-ranked candidates are refined whatever the window (HMP_REFINE_MIN_LEADERS)
 	int refine_rounds = 2;           // HMP_REFINE_ROUNDS=1 in the environment: first round only (A/B)
 	int refine_window_only = 0;      // HMP_REFINE_WINDOW_ONLY=1: round 1 by the relative window (the r01 rule) instead of by rank (A/B)
+	std::vector<HmpSceneCosts> scene_costs;   // per-scene scales / shifts of hmp_plan_batch (hmp_set_scene_costs); empty: shared params
 	HmpEquisampled equi{};           // second generator of the pool (hmp_set_equisampled); enabled = 0 after hmp_create
 	std::vector<double> last_equi;   // its velocity samples of the last plan ([n][3])
 	bool dilated_dirty = true;       // costmap cells, footprint or separation changed since the dilated map was built
@@ -226,6 +227,7 @@ struct HmpContext {
 	int n_seeds[HMP_NUM_MAPGRIDS] = {0, 0, 0, 0};
 	DevBuf d_params, d_amp, d_extra, d_scenes, d_costmaps, d_mapgrids, d_totals, d_block_best, d_ctrl, d_detail, d_dbg, d_refine, d_dilated, d_equi, d_env, d_mask, d_hvrec, d_posescr, d_poseslots;
 	HostBuf h_stage, h_out;
+	HostBuf h_params;  // pinned staging of the per-scene DevParams copies of a batch with a cost table
 	HostBuf h_small;   // pinned words read back inside a cycle: [0..3] overflow status of the four wave fronts, [4..5] leader counts
 	HostBuf h_grid[HMP_NUM_MAPGRIDS];   // pinned staging of hmp_set_mapgrid, one per slot
 	uint32_t costmap_stride = 0;
@@ -234,6 +236,7 @@ struct HmpContext {
 	int last_n_candidates = 0, last_T = 0, last_n_scenes = 0;
 	uint32_t last_scene_stride = 0;
 	DevParams last_dev_params{};
+	std::vector<HmpSceneCosts> last_scene_costs;   // the table the last plan ran with (empty: none)
 	std::vector<double> last_amp_table;
 	std::vector<HmpSample> last_extra;
 	bool last_valid = false;
@@ -647,7 +650,17 @@ struct PlanLaunch {
 	uint32_t scene_stride;
 	int n_extra;
 	int T;
+	const HmpSceneCosts* scene_costs = nullptr;   // n_scenes entries (hmp_set_scene_costs), or null: every scene uses D's
 };
+
+// Whether critic k is evaluated in any scene of a launch: host decisions that serve all scenes at once (inputs the critic
+// needs, shared-memory reservations) follow the union over the scenes; the kernels skip the critic per scene.
+bool scale_on(const double* shared_scale, const HmpSceneCosts* scene_costs, int n_scenes, int k) {
+	if (!scene_costs) return shared_scale[k] != 0.0;
+	for (int s = 0; s < n_scenes; ++s)
+		if (scene_costs[s].scale[k] != 0.0) return true;
+	return false;
+}
 
 int launch_main(HmpContext* ctx, const DevParams& D, const PlanLaunch& pl, int* blocks_x_out, size_t* smem_out,
                 int* costmap_in_smem_out, int* sweep_mode_out = nullptr, size_t* smem_sweep_out = nullptr) {
@@ -702,7 +715,7 @@ int launch_main(HmpContext* ctx, const DevParams& D, const PlanLaunch& pl, int* 
 			smem_sweep = smem;
 		}
 	}
-	if (tpc_threads && ctx->prune_obstacle && D.scale[HMP_COST_OBSTACLE] != 0.0 && D.n_footprint > 0 && !D.occdist_sum &&
+	if (tpc_threads && ctx->prune_obstacle && scale_on(D.scale, pl.scene_costs, pl.n_scenes, HMP_COST_OBSTACLE) && D.n_footprint > 0 && !D.occdist_sum &&
 	    !getenv("HMP_NO_DEFER")) {
 		// deferred obstacle critic: one byte per pose and thread behind the packed static objects; taken when it costs no
 		// resident block (the pose scratch in global memory is one slot per resident block, run_cycle)
@@ -850,6 +863,7 @@ void hmp_destroy(HmpContext* ctx) {
 	                  &ctx->d_totals, &ctx->d_block_best, &ctx->d_ctrl, &ctx->d_detail, &ctx->d_dbg, &ctx->d_refine, &ctx->d_dilated, &ctx->d_equi, &ctx->d_env, &ctx->d_mask, &ctx->d_hvrec, &ctx->d_posescr, &ctx->d_poseslots};
 	for (DevBuf* b : bufs) b->release();
 	ctx->h_stage.release();
+	ctx->h_params.release();
 	for (int b = 0; b < 2; ++b) {
 		ctx->h_grid_stage[b].release();
 		if (ctx->grid_stage_ev[b]) cudaEventDestroy(ctx->grid_stage_ev[b]);
@@ -1242,7 +1256,10 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 	const int T = D.T;
 	const int NS = pl.n_scenes;
 	int rc;
-	if ((rc = ctx->d_params.ensure(sizeof(DevParams)))) return rc;
+	// with a per-scene cost table: one DevParams per scene, D with that scene's scales / shifts (scene 0 first, so that launches
+	// that read the first block, e.g. hmp_explain after a one-scene batch, see scene 0's values)
+	const size_t params_bytes = sizeof(DevParams) * (pl.scene_costs ? (size_t)NS : 1);
+	if ((rc = ctx->d_params.ensure(params_bytes))) return rc;
 	if ((rc = ctx->d_amp.ensure(amp_table.size() * sizeof(double)))) return rc;
 	if ((rc = ctx->d_extra.ensure(std::max<size_t>(1, (size_t)n_extra) * sizeof(HmpSample)))) return rc;
 	if ((rc = ctx->d_equi.ensure(std::max<size_t>(1, equi.size()) * sizeof(double)))) return rc;
@@ -1269,7 +1286,21 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 	if ((rc = ctx->d_block_best.ensure((size_t)NS * ((size_t)blocks_x + equi_blocks) * 2 * sizeof(unsigned long long)))) return rc;
 
 	cudaStream_t st = ctx->stream;
-	CU(cudaMemcpyAsync(ctx->d_params.p, &D, sizeof(DevParams), cudaMemcpyHostToDevice, st));
+	if (pl.scene_costs) {
+		if ((rc = ctx->h_params.ensure(params_bytes))) return rc;
+		CU(cudaStreamSynchronize(st));   // no copy from the staging buffer is still in flight
+		DevParams* hp = (DevParams*)ctx->h_params.p;
+		for (int s = 0; s < NS; ++s) {
+			const HmpSceneCosts& sc = pl.scene_costs[s];
+			hp[s] = D;
+			std::memcpy(hp[s].scale, sc.scale, sizeof(hp[s].scale));
+			std::memcpy(hp[s].mg_xshift, sc.xshift, sizeof(hp[s].mg_xshift));
+			std::memcpy(hp[s].mg_yshift, sc.yshift, sizeof(hp[s].mg_yshift));
+		}
+		CU(cudaMemcpyAsync(ctx->d_params.p, hp, params_bytes, cudaMemcpyHostToDevice, st));
+	} else {
+		CU(cudaMemcpyAsync(ctx->d_params.p, &D, sizeof(DevParams), cudaMemcpyHostToDevice, st));
+	}
 	CU(cudaMemcpyAsync(ctx->d_amp.p, amp_table.data(), amp_table.size() * sizeof(double), cudaMemcpyHostToDevice, st));
 	if (n_extra > 0) CU(cudaMemcpyAsync(ctx->d_extra.p, extra, (size_t)n_extra * sizeof(HmpSample), cudaMemcpyHostToDevice, st));
 	if (!equi.empty()) CU(cudaMemcpyAsync(ctx->d_equi.p, equi.data(), equi.size() * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -1279,6 +1310,7 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 	KernelArgs A;
 	std::memset(&A, 0, sizeof(A));
 	A.params = (const DevParams*)ctx->d_params.p;
+	A.params_stride = pl.scene_costs ? (uint32_t)sizeof(DevParams) : 0u;
 	A.amp_values = (const double*)ctx->d_amp.p;
 	A.extra_samples = (const double*)ctx->d_extra.p;
 	A.equi_samples = (const double*)ctx->d_equi.p;
@@ -1309,7 +1341,7 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 
 	CU(cudaEventRecord(ctx->ev0, st));
 	// dilated max-cost map for the exact pruning of the obstacle critic (rebuilt when costmap / footprint / separation change)
-	if (ctx->prune_obstacle && D.scale[HMP_COST_OBSTACLE] != 0.0 && D.n_footprint > 0) {
+	if (ctx->prune_obstacle && scale_on(D.scale, pl.scene_costs, NS, HMP_COST_OBSTACLE) && D.n_footprint > 0) {
 		if (ctx->dilated_dirty || ctx->dilated_scenes != NS) {
 			if ((rc = ctx->d_dilated.ensure((size_t)ctx->costmap_stride * NS))) return rc;
 			double r_fp = 0.0, r_k = 0.0;
@@ -1620,6 +1652,8 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 	ctx->last_n_scenes = NS;
 	ctx->last_scene_stride = pl.scene_stride;
 	ctx->last_dev_params = D;
+	if (!pl.scene_costs) ctx->last_scene_costs.clear();
+	else if (pl.scene_costs != ctx->last_scene_costs.data()) ctx->last_scene_costs.assign(pl.scene_costs, pl.scene_costs + NS);
 	if (&amp_table != &ctx->last_amp_table) ctx->last_amp_table = amp_table;
 	if (extra != ctx->last_extra.data()) ctx->last_extra.assign(extra, extra + n_extra);
 	if (&equi != &ctx->last_equi) ctx->last_equi = equi;
@@ -1845,7 +1879,13 @@ int hmp_plan_batch(HmpContext* ctx, const HmpWorld* worlds, int32_t n_scenes, co
 		set_err("bad batch arguments");
 		return HMP_E_INVALID;
 	}
-	if (!ctx->have_footprint && ctx->params.costs.scale[HMP_COST_OBSTACLE] != 0.0) {
+	if (!ctx->scene_costs.empty() && (size_t)n_scenes > ctx->scene_costs.size()) {
+		set_err("the per-scene cost table holds %zu scenes, the batch has %d", ctx->scene_costs.size(), n_scenes);
+		return HMP_E_INVALID;
+	}
+	const HmpSceneCosts* table = ctx->scene_costs.empty() ? nullptr : ctx->scene_costs.data();
+	const double* scale = ctx->params.costs.scale;
+	if (!ctx->have_footprint && scale_on(scale, table, n_scenes, HMP_COST_OBSTACLE)) {
 		set_err("hmp_set_footprint has not been called");
 		return HMP_E_NOT_READY;
 	}
@@ -1878,7 +1918,7 @@ int hmp_plan_batch(HmpContext* ctx, const HmpWorld* worlds, int32_t n_scenes, co
 		}
 	} else {
 		for (int g = 0; g < HMP_NUM_MAPGRIDS; ++g) {
-			if (ctx->params.costs.scale[HMP_COST_PATH + g] == 0.0) continue;
+			if (!scale_on(scale, table, n_scenes, HMP_COST_PATH + g)) continue;
 			if (n_scenes == 1 ? !ctx->have_grid[g] : ctx->batch_grid_scenes < n_scenes) {
 				set_err("MapGrid %d is not resident for %d scene(s): pass target_dist or call hmp_compute_mapgrid_batch / hmp_set_mapgrids_batch_f32 first", g,
 				        n_scenes);
@@ -2001,7 +2041,7 @@ int hmp_plan_batch(HmpContext* ctx, const HmpWorld* worlds, int32_t n_scenes, co
 		for (bool& b : ctx->have_grid) b = true;
 		ctx->batch_grid_scenes = n_scenes;
 	}
-	PlanLaunch pl{n_scenes, (uint32_t)stride, 0, T};
+	PlanLaunch pl{n_scenes, (uint32_t)stride, 0, T, table};
 	return run_cycle(ctx, D, amp_table, nullptr, 0, equi_all, pl, results, nullptr, 0);
 }
 
@@ -2017,7 +2057,8 @@ int hmp_replan_resident(HmpContext* ctx, HmpResult* results, int32_t results_cap
 		return HMP_E_INVALID;
 	}
 	CU(cudaSetDevice(ctx->device));
-	PlanLaunch pl{ctx->last_n_scenes, ctx->last_scene_stride, (int)ctx->last_extra.size(), ctx->last_T};
+	PlanLaunch pl{ctx->last_n_scenes, ctx->last_scene_stride, (int)ctx->last_extra.size(), ctx->last_T,
+	              ctx->last_scene_costs.empty() ? nullptr : ctx->last_scene_costs.data()};
 	return run_cycle(ctx, ctx->last_dev_params, ctx->last_amp_table, pl.n_extra ? ctx->last_extra.data() : nullptr, pl.n_extra,
 	                 ctx->last_equi, pl, results, nullptr, 0);
 }
@@ -2592,6 +2633,27 @@ int hmp_set_equisampled(HmpContext* ctx, const HmpEquisampled* eq) {
 	if (eq) ctx->equi = *eq;
 	else ctx->equi.enabled = 0;
 	ctx->last_valid = false;
+	return HMP_OK;
+}
+
+int hmp_set_scene_costs(HmpContext* ctx, const HmpSceneCosts* costs, int32_t n_scenes) {
+	if (!ctx || n_scenes < 0 || (n_scenes > 0 && !costs)) {
+		set_err("bad scene cost arguments (null context, negative count or null table)");
+		return HMP_E_INVALID;
+	}
+	if (!costs || n_scenes == 0) {
+		ctx->scene_costs.clear();
+		return HMP_OK;
+	}
+	for (int s = 0; s < n_scenes; ++s) {
+		const double* v = (const double*)&costs[s];
+		for (size_t i = 0; i < sizeof(HmpSceneCosts) / sizeof(double); ++i)
+			if (!std::isfinite(v[i])) {
+				set_err("scene %d: non-finite scale or shift", s);
+				return HMP_E_INVALID;
+			}
+	}
+	ctx->scene_costs.assign(costs, costs + n_scenes);
 	return HMP_OK;
 }
 

@@ -173,7 +173,7 @@ struct alignas(16) DevParams {
 
 /* Kernel argument block (passed by value). */
 struct KernelArgs {
-	const DevParams* params;         /* device */
+	const DevParams* params;         /* device; scene s reads the block params_stride * s bytes further on */
 	const double* amp_values;        /* [10][HMP_MAX_AMP_VALUES] device                           */
 	const double* extra_samples;     /* [n_extra][10] device, or null                             */
 	const double* equi_samples;      /* [n_scenes][n_equi][3] target velocities (float values), or null */
@@ -229,7 +229,7 @@ struct KernelArgs {
 	 * pose_n_slots >= blocks that can be resident at once, so a free slot always exists. */
 	unsigned int* pose_slots;
 	int32_t pose_n_slots;
-	int32_t _padp;
+	uint32_t params_stride;          /* 0: one DevParams for every scene; sizeof(DevParams): one per scene (hmp_set_scene_costs) */
 };
 
 #endif

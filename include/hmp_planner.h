@@ -406,7 +406,8 @@ int hmp_plan(HmpContext* ctx, const HmpWorld* world, const HmpSampling* sampling
              HmpResult* result, double* poses_out, int32_t poses_capacity);
 
 /* Same, for a batch of independent scenes that share params, costmap geometry and sampling but
- * have their own world, costmap cells and MapGrids (BASELINE config "batched scenes"). Scene s uses
+ * have their own world, costmap cells and MapGrids (BASELINE config "batched scenes"); with hmp_set_scene_costs each scene
+ * also has its own critic scales and MapGrid shifts. Scene s uses
  * worlds[s], cells + s * size_x * size_y, target_dist[g] + s * size_x * size_y. One launch.
  * cells = NULL reuses the costmaps of an earlier batch call, target_dist = NULL the grids left resident by
  * hmp_compute_mapgrid_batch / hmp_set_mapgrids_batch_f32 / an earlier batch; HMP_E_NOT_READY / HMP_E_INVALID if they do
@@ -434,6 +435,21 @@ int hmp_set_mapgrids_batch_f32(HmpContext* ctx, int32_t n_scenes, const float* c
  * from it run asynchronously at the full PCIe rate (the driver stages copies from pageable memory). NULL on failure. */
 void* hmp_host_alloc(size_t bytes);
 void hmp_host_free(void* p);
+
+/* Per-world values of the per-cycle setScale / setXShift / setYShift calls (updateLocalCosts, humap_planner.cpp:1054-1141):
+ * each robot of a batch derives them from its own state (distance to its goal, gap to the nearest person, goal inside a
+ * group). */
+typedef struct HmpSceneCosts {
+	double scale[HMP_NUM_COSTS];      /* same meaning as HmpCosts.scale (MapGrid scales already x resolution); 0 skips the critic */
+	double xshift[HMP_NUM_MAPGRIDS];  /* same meaning as HmpCosts.xshift / yshift                                               */
+	double yshift[HMP_NUM_MAPGRIDS];
+} HmpSceneCosts;
+/* Sets the per-scene cost table of the following hmp_plan_batch calls: scene s uses costs[s] in place of HmpCosts.scale /
+ * xshift / yshift; every other field of HmpParams stays shared. The table is copied. costs = NULL or n_scenes = 0 clears it,
+ * which is the state after hmp_create. hmp_set_params does not clear it; hmp_plan ignores it; hmp_plan_batch with more
+ * scenes than the table holds returns HMP_E_INVALID; hmp_replan_resident re-runs with the table the last plan used.
+ * HMP_E_INVALID for a negative count, a NULL table with n_scenes > 0 or a non-finite value. */
+int hmp_set_scene_costs(HmpContext* ctx, const HmpSceneCosts* costs, int32_t n_scenes);
 
 /* Re-runs the last hmp_plan / hmp_plan_batch on the scene data still resident in device memory (only
  * the few-KB parameter block is re-sent and the result read back). `results` must hold results_capacity >=
