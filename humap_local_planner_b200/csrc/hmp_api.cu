@@ -172,7 +172,6 @@ struct HmpContext {
 	cudaStream_t stream = nullptr;
 	cudaStream_t stream2 = nullptr;   // FP64 rollouts of a small pool, beside the FP32 sweep (run_cycle)
 	cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-	int overlap_refine = 1;           // HMP_NO_OVERLAP=1 in the environment: the refinement follows the sweep (A/B)
 	cudaEvent_t ev0 = nullptr, ev1 = nullptr, evm = nullptr;
 	int64_t launches = 0;
 
@@ -201,9 +200,6 @@ struct HmpContext {
 	int escalate_min = 24;          // hmp_set_escalation: from this many unreliable leaders the plan is redone in FP64 (0: never)
 	int last_escalated = 0;         // the last plan was redone in FP64 for that reason
 	int last_fallback_rounds = 0;   // extra refinement rounds of the last plan because FP64 rejected every leader (mode 2)
-	int refine_min_leaders = 16;     // the best-ranked candidates are refined whatever the window (HMP_REFINE_MIN_LEADERS)
-	int refine_rounds = 2;           // HMP_REFINE_ROUNDS=1 in the environment: first round only (A/B)
-	int refine_window_only = 0;      // HMP_REFINE_WINDOW_ONLY=1: round 1 by the relative window (the r01 rule) instead of by rank (A/B)
 	std::vector<HmpSceneCosts> scene_costs;   // per-scene scales / shifts of hmp_plan_batch (hmp_set_scene_costs); empty: shared params
 	HmpEquisampled equi{};           // second generator of the pool (hmp_set_equisampled); enabled = 0 after hmp_create
 	std::vector<double> last_equi;   // its velocity samples of the last plan ([n][3])
@@ -668,7 +664,7 @@ int launch_main(HmpContext* ctx, const DevParams& D, const PlanLaunch& pl, int* 
 	size_t cm_bytes = (size_t)ctx->costmap_stride;
 	int in_smem = 1;
 	size_t smem = hmp_dev_smem_bytes(pl.scene_stride, (uint32_t)cm_bytes, 1);
-	if (smem > ctx->max_smem_optin || cm_bytes > (1u << 19) || getenv("HMP_CM_GLOBAL")) {   // HMP_CM_GLOBAL=1: A/B of the global-memory costmap path
+	if (smem > ctx->max_smem_optin || cm_bytes > (1u << 19)) {
 		in_smem = 0;
 		smem = hmp_dev_smem_bytes(pl.scene_stride, (uint32_t)cm_bytes, 0);
 		if (smem > ctx->max_smem_optin) {
@@ -680,10 +676,10 @@ int launch_main(HmpContext* ctx, const DevParams& D, const PlanLaunch& pl, int* 
 	// candidates; one thread per candidate (sweep_tpc_kernel) issues the per-step scalar section once per 32 candidates
 	// and wins as soon as the launch holds enough candidates to give every SM sub-partition a warp.
 	// The exact-parity sweep (precision mode 1) has the same two layouts; its thread-per-candidate instance is compiled for one
-	// block per SM (225 registers, no spills). HMP_F64_WARP=1 keeps the warp-per-candidate FP64 sweep (A/B).
+	// block per SM (225 registers, no spills).
 	int tpc_threads = 0;
 	const bool f64 = ctx->precise == 1;
-	if (sweep_mode_out && !(f64 && getenv("HMP_F64_WARP"))) {
+	if (sweep_mode_out) {
 		const long long total = (long long)C * pl.n_scenes;
 		const bool want = ctx->sweep_layout == 2 || (ctx->sweep_layout == 0 && total >= 16384);
 		if (want) {
@@ -693,19 +689,7 @@ int launch_main(HmpContext* ctx, const DevParams& D, const PlanLaunch& pl, int* 
 				tpc_threads = (tpc_threads > 128) ? 128 : 64;
 		}
 	}
-	if (tpc_threads && !f64) {
-		if (const char* e = getenv("HMP_TPC_LAUNCH_THREADS")) {   // A/B: block size of the FP32 thread-per-candidate sweep
-			const int v = atoi(e);
-			if (v >= 32 && v <= hmp_dev_tpc_max_threads() && v % 32 == 0) tpc_threads = v;
-		}
-	}
-	if (tpc_threads && f64) {
-		// finer tickets balance the two rounds a 64k grid takes at 8 warps per SM (rejected candidates end early)
-		const char* e = getenv("HMP_F64_TPC_THREADS");
-		const int v = e ? atoi(e) : hmp_dev_tpc64_max_threads();
-		tpc_threads = std::min(tpc_threads, hmp_dev_tpc64_max_threads());
-		if (v >= 32 && v <= hmp_dev_tpc64_max_threads() && v % 32 == 0) tpc_threads = std::min(tpc_threads, v);
-	}
+	if (tpc_threads && f64) tpc_threads = std::min(tpc_threads, hmp_dev_tpc64_max_threads());   // launch bound of the FP64 instance
 	size_t smem_sweep = smem;
 	ctx->tpc_defer = 0;
 	if (tpc_threads) {
@@ -715,27 +699,25 @@ int launch_main(HmpContext* ctx, const DevParams& D, const PlanLaunch& pl, int* 
 			smem_sweep = smem;
 		}
 	}
+	// few warps per SM sub-partition anyway (<= 2): the register-rich instance of the thread-per-candidate sweep
+	int tpc_rich = 0;
+	if (tpc_threads && !f64) {
+		const long long warps = (((long long)C + tpc_threads - 1) / tpc_threads) * pl.n_scenes * (tpc_threads / 32);
+		tpc_rich = (warps <= (long long)ctx->sm_count * 8) ? 1 : 0;
+	}
 	if (tpc_threads && ctx->prune_obstacle && scale_on(D.scale, pl.scene_costs, pl.n_scenes, HMP_COST_OBSTACLE) && D.n_footprint > 0 && !D.occdist_sum &&
 	    !getenv("HMP_NO_DEFER")) {
 		// deferred obstacle critic: one byte per pose and thread behind the packed static objects; taken when it costs no
 		// resident block (the pose scratch in global memory is one slot per resident block, run_cycle)
 		const size_t with = ((smem_sweep + 15) & ~(size_t)15) + (size_t)pl.T * tpc_threads;
 		int b0 = 0, b1 = 0;
-		const long long warps = (((long long)C + tpc_threads - 1) / tpc_threads) * pl.n_scenes * (tpc_threads / 32);
-		const int rich = (warps <= (long long)ctx->sm_count * 8 && !getenv("HMP_TPC_NO_RICH")) ? 1 : 0;
 		auto occ = [&](size_t bytes, int* b) {
-			return f64 ? hmp_dev_occupancy_tpc64(bytes, tpc_threads, b) : hmp_dev_occupancy_tpc(bytes, tpc_threads, rich, b);
+			return f64 ? hmp_dev_occupancy_tpc64(bytes, tpc_threads, b) : hmp_dev_occupancy_tpc(bytes, tpc_threads, tpc_rich, b);
 		};
 		if (with <= ctx->max_smem_optin && occ(smem_sweep, &b0) == cudaSuccess && occ(with, &b1) == cudaSuccess && b1 >= b0 && b1 >= 1) {
 			smem_sweep = with;
 			ctx->tpc_defer = 1;
 		}
-	}
-	// few warps per SM sub-partition anyway (<= 2): the register-rich instance of the thread-per-candidate sweep
-	int tpc_rich = 0;
-	if (tpc_threads && !f64) {
-		const long long warps = (((long long)C + tpc_threads - 1) / tpc_threads) * pl.n_scenes * (tpc_threads / 32);
-		tpc_rich = (warps <= (long long)ctx->sm_count * 8 && !getenv("HMP_TPC_NO_RICH")) ? 1 : 0;
 	}
 	int bps = 0;
 	if (tpc_threads && f64) CU(hmp_dev_occupancy_tpc64(smem_sweep, tpc_threads, &bps));
@@ -811,10 +793,6 @@ HmpContext* hmp_create(int device_id) {
 	}
 	ctx->device = device_id;
 	ctx->prune_obstacle = getenv("HMP_NO_PRUNE") ? 0 : 1;
-	if (const char* e = getenv("HMP_REFINE_MIN_LEADERS")) ctx->refine_min_leaders = std::max(1, std::min(256, atoi(e)));
-	if (const char* e = getenv("HMP_REFINE_ROUNDS")) ctx->refine_rounds = std::max(1, std::min(2, atoi(e)));
-	if (getenv("HMP_REFINE_WINDOW_ONLY")) ctx->refine_window_only = 1;
-	if (getenv("HMP_NO_OVERLAP")) ctx->overlap_refine = 0;
 	if (const char* e = getenv("HMP_ESCALATE")) ctx->escalate_min = std::max(0, atoi(e));
 	if (const char* e = getenv("HMP_SWEEP_LAYOUT")) ctx->sweep_layout = std::max(0, std::min(2, atoi(e)));
 	ctx->sm_count = prop.multiProcessorCount;
@@ -1387,7 +1365,7 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 	// whatever the FP32 sweep says, so the FP64 rollouts do not depend on it and run BESIDE it on a second stream; the FP32
 	// sweep still supplies the counters and the highest_valid_cost_ records. (K as in the refinement below.)
 	const int k_all = std::max(8, (C + 7) / 8 * 8);
-	const bool overlap = ctx->precise == 2 && NS == 1 && ctx->overlap_refine && !ctx->refine_window_only && ctx->refine_max_leaders <= 0 &&
+	const bool overlap = ctx->precise == 2 && NS == 1 && ctx->refine_max_leaders <= 0 &&
 	                     k_all + blocks_x + equi_blocks <= ctx->sm_count;
 	if (overlap) {
 		CU(cudaEventRecord(ctx->ev_fork, st));   // inputs of the cycle are on the device (uploads, wave fronts, dilated map)
@@ -1437,9 +1415,10 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 		const size_t r_set = (r_bytes + 15) / 16 * 16;
 		// single-scene plans run a second round (below): a second set of buffers + the first round's threshold
 		// (not when round 1 already holds every candidate of the pool, C <= K: nothing is left for a second list)
-		const int rounds = (NS == 1 && ctx->refine_rounds >= 2 && (C > K || ctx->refine_window_only)) ? 2 : 1;
+		const int rounds = (NS == 1 && C > K) ? 2 : 1;
 		if ((rc = ctx->d_refine.ensure(r_set * rounds + 2 * NS * sizeof(double)))) return rc;   // + (threshold, effective window) of round 1
 		double* r_thr = (double*)((unsigned char*)ctx->d_refine.p + r_set * rounds);
+		constexpr int REFINE_MIN_LEADERS = 16;   // collect_leaders_kernel: the best-ranked candidates a window-based FIRST round always lists
 		refine_round = [=, &r_count_dev](int round, const int32_t* active) -> int {
 			unsigned char* base = (unsigned char*)ctx->d_refine.p + r_set * round;
 			double* r_costs = (double*)base;
@@ -1456,11 +1435,11 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 			cudaStream_t rs = beside ? ctx->stream2 : st;
 			if (beside)
 				CU(hmp_dev_launch_fill_leaders(r_leaders, K, C, r_count, rs));
-			else if (round == 0 && !ctx->refine_window_only)
+			else if (round == 0)
 				CU(hmp_dev_launch_collect_topk(A.totals, C, A.best_out, K, ctx->refine_window, r_leaders, r_count, r_thr, NS, active, st));
 			else
-				CU(hmp_dev_launch_collect_leaders(A.totals, C, A.best_out, ctx->refine_window, K, r_leaders, r_count,
-				                                  round ? r_thr : nullptr, round ? nullptr : r_thr, ctx->refine_min_leaders, NS, active, st));
+				CU(hmp_dev_launch_collect_leaders(A.totals, C, A.best_out, ctx->refine_window, K, r_leaders, r_count, r_thr, nullptr,
+				                                  REFINE_MIN_LEADERS, NS, active, st));
 			KernelArgs Rf = A;
 			Rf.hv_pre = nullptr;
 			Rf.hv_val = nullptr;

@@ -19,21 +19,8 @@
 #define HMP_WARPS_PER_BLOCK 8
 #endif
 #define HMP_THREADS_PER_BLOCK (32 * HMP_WARPS_PER_BLOCK)
-#ifndef HMP_LOCKSTEP
-#define HMP_LOCKSTEP 1
-#endif
-#ifndef HMP_LOCKSTEP_PERIOD
-#define HMP_LOCKSTEP_PERIOD 1   /* steps between two block barriers of the lockstep rollout */
-#endif
-#ifndef HMP_LOCKSTEP_EXTRA
-#define HMP_LOCKSTEP_EXTRA 0
-#endif
 #ifndef HMP_MIN_BLOCKS
 #define HMP_MIN_BLOCKS 2
-#endif
-#ifndef HMP_F64_FAST
-#define HMP_F64_FAST 1   /* 1: FP64 object loops with rsqrt-based lengths and one merged exponential per static object (ulp-level
-                            differences from the literal form; cfg2 exact-mode sweep 56.0 -> 51.6 ms, r02d A/B); 0: the literal form */
 #endif
 #ifndef HMP_F64_STATIC_UNROLL
 #define HMP_F64_STATIC_UNROLL 2   /* static objects in flight per lane in the FP64 instances */
