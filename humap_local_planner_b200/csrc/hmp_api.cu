@@ -69,13 +69,9 @@ extern "C" cudaError_t hmp_dev_launch_world_to_map(const DevParams* P, const dou
                                                    int* my, int* ok, cudaStream_t stream);
 extern "C" cudaError_t hmp_dev_launch_footprint_cost(const DevParams* P, const uint8_t* cm, const double* xyt, int n,
                                                      double* cost, cudaStream_t stream);
-extern "C" cudaError_t hmp_dev_launch_wavefront(const uint8_t* cm, int sx, int sy, const int* seeds, int n_seeds, float* dist,
-                                                cudaStream_t stream);
-extern "C" cudaError_t hmp_dev_launch_wavefront_queue(const uint8_t* cm, int sx, int sy, const int* seeds, int n_seeds, float* dist,
-                                                      int* status, cudaStream_t stream);
-extern "C" size_t hmp_dev_wavefront_smem(int sx, int sy, int queue);
-extern "C" cudaError_t hmp_dev_launch_wavefront_batch(const uint8_t* cms, uint32_t cm_stride, int sx, int sy, const int* seeds,
-                                                      const int* seed_off, float* dist, int* status, int n_scenes, cudaStream_t stream);
+extern "C" size_t hmp_dev_wavefront_smem(int sx, int sy);
+extern "C" cudaError_t hmp_dev_launch_wavefront(const uint8_t* cms, uint32_t cm_stride, int sx, int sy, const int* seeds,
+                                                const int* seed_off, float* dist, int n_grids, int n_scenes, cudaStream_t stream);
 extern "C" cudaError_t hmp_dev_launch_fis(const double* in4, int n, double* out2, int precise, cudaStream_t stream);
 extern "C" cudaError_t hmp_dev_launch_ffma_peak(int blocks, int iters, float* sink, cudaStream_t stream);
 extern "C" cudaError_t hmp_dev_launch_cost_cloud(const DevParams* P, int n_cells, const uint8_t* cm, const float* mapgrids, const double* hv,
@@ -186,7 +182,6 @@ struct HmpContext {
 	std::vector<uint8_t> h_cells;   // host copy of the single-scene costmap (scene 0 after a batch): seed test of the device wave front
 	int costmap_scenes = 0;         // scenes whose costmap is resident in d_costmaps (1 after hmp_set_costmap, n after a batch upload)
 	int batch_grid_scenes = 0;      // scenes whose four MapGrids are resident in d_mapgrids from a batch call (0: single-scene slots only)
-	int batch_wf_pending = 0;       // scenes of a hmp_compute_mapgrid_batch whose wave fronts still run on wf_stream[0] (0: none)
 	bool have_footprint = false;
 	int precise = 2;                 // 0 FP32, 1 FP64, 2 (default) FP32 sweep + FP64 refinement of the leaders
 	double refine_window = 0.02;     // leaders: FP32 total <= best * (1 + window)
@@ -219,12 +214,14 @@ struct HmpContext {
 	cudaStream_t wf_stream[HMP_NUM_MAPGRIDS] = {nullptr, nullptr, nullptr, nullptr};   // the four wave fronts of a cycle run side by side
 	cudaEvent_t wf_done[HMP_NUM_MAPGRIDS] = {nullptr, nullptr, nullptr, nullptr};
 	bool seeds_event_valid[HMP_NUM_MAPGRIDS] = {false, false, false, false};
-	bool wavefront_pending[HMP_NUM_MAPGRIDS] = {false, false, false, false};
-	int n_seeds[HMP_NUM_MAPGRIDS] = {0, 0, 0, 0};
+	bool wavefront_pending[HMP_NUM_MAPGRIDS] = {false, false, false, false};   // slot 0 also stands for a hmp_compute_mapgrid_batch
+	// wf_done[g] was last recorded by a batch of wave fronts (on wf_stream[0]), which writes slot g too: the next single-grid wave
+	// front of the slot waits for it on the device. A join does not clear this, it orders ctx->stream only.
+	bool wf_after_batch[HMP_NUM_MAPGRIDS] = {false, false, false, false};
 	DevBuf d_params, d_amp, d_extra, d_scenes, d_costmaps, d_mapgrids, d_totals, d_block_best, d_ctrl, d_detail, d_dbg, d_refine, d_dilated, d_equi, d_env, d_mask, d_hvrec, d_posescr, d_poseslots;
 	HostBuf h_stage, h_out;
 	HostBuf h_params;  // pinned staging of the per-scene DevParams copies of a batch with a cost table
-	HostBuf h_small;   // pinned words read back inside a cycle: [0..3] overflow status of the four wave fronts, [4..5] leader counts
+	HostBuf h_small;   // pinned words read back inside a cycle: [0..1] leader counts of the two refinement rounds, [2] unreliable leaders
 	HostBuf h_grid[HMP_NUM_MAPGRIDS];   // pinned staging of hmp_set_mapgrid, one per slot
 	uint32_t costmap_stride = 0;
 
@@ -879,7 +876,16 @@ int hmp_set_params(HmpContext* ctx, const HmpParams* params) {
 	return HMP_OK;
 }
 
-static int resolve_wavefronts(HmpContext* ctx);
+// Device wave fronts (hmp_compute_mapgrid[_batch]) run on side streams and finish on the device whatever their frontiers hold:
+// the plan stream waits for their events, the host does not. Work queued on ctx->stream after the join sees their grids.
+static int join_wavefronts(HmpContext* ctx) {
+	for (int g = 0; g < HMP_NUM_MAPGRIDS; ++g) {
+		if (!ctx->wavefront_pending[g]) continue;
+		CU(cudaStreamWaitEvent(ctx->stream, ctx->wf_done[g], 0));
+		ctx->wavefront_pending[g] = false;
+	}
+	return HMP_OK;
+}
 
 int hmp_set_costmap(HmpContext* ctx, const uint8_t* cells, int32_t size_x, int32_t size_y, double origin_x, double origin_y,
                     double resolution) {
@@ -892,10 +898,6 @@ int hmp_set_costmap(HmpContext* ctx, const uint8_t* cells, int32_t size_x, int32
 		return HMP_E_CAPACITY;
 	}
 	CU(cudaSetDevice(ctx->device));
-	if (ctx->batch_wf_pending) {   // a batch of wave fronts still reading the old cells must finish first
-		int rcw = resolve_wavefronts(ctx);
-		if (rcw) return rcw;
-	}
 	for (int g = 0; g < HMP_NUM_MAPGRIDS; ++g)   // a wave front still reading the old cells must finish first
 		if (ctx->wavefront_pending[g]) CU(cudaStreamSynchronize(ctx->wf_stream[g]));
 	if (size_x != ctx->size_x || size_y != ctx->size_y) {
@@ -939,20 +941,14 @@ int hmp_set_mapgrid(HmpContext* ctx, int32_t grid, const double* target_dist, do
 		return HMP_E_NOT_READY;
 	}
 	CU(cudaSetDevice(ctx->device));
-	if (ctx->batch_wf_pending) {
-		int rcw = resolve_wavefronts(ctx);
-		if (rcw) return rcw;
-	}
-	if (ctx->wavefront_pending[grid]) {   // an uploaded grid replaces a device wave front still in flight for this slot
-		CU(cudaStreamSynchronize(ctx->wf_stream[grid]));
-		ctx->wavefront_pending[grid] = false;
-	}
+	int rc = join_wavefronts(ctx);   // the upload lands after any device wave front still writing this slot
+	if (rc) return rc;
 	size_t n = (size_t)ctx->size_x * ctx->size_y;
 	// one pinned staging buffer per slot: the four uploads of a cycle queue on the stream without a host synchronisation
 	// (the previous cycle's plan has synchronised, so the buffer is free); the conversion loop is branch-free so that the
 	// host compiler vectorises it (it used to be a third of the e2e overhead of a cycle)
 	if (n * sizeof(float) > ctx->h_grid[grid].cap) CU(cudaStreamSynchronize(ctx->stream));
-	int rc = ctx->h_grid[grid].ensure(n * sizeof(float));
+	rc = ctx->h_grid[grid].ensure(n * sizeof(float));
 	if (rc) return rc;
 	float* f = (float*)ctx->h_grid[grid].p;
 	const double limit = (double)n + 1.0;
@@ -977,94 +973,6 @@ int hmp_set_mapgrid(HmpContext* ctx, int32_t grid, const double* target_dist, do
 	ctx->batch_grid_scenes = 0;
 	ctx->hv_prev[grid] = highest_valid_cost_prev;
 	ctx->last_valid = false;
-	return HMP_OK;
-}
-
-
-// Checks the overflow flag of queued wave fronts; a grid whose frontier overflowed the shared-memory queues is recomputed
-// with the scan kernel (never observed for 200 x 200 windows; kept for correctness on pathological maps).
-static int resolve_wavefronts(HmpContext* ctx) {
-	if (ctx->batch_wf_pending > 0) {
-		// batch of wave fronts (hmp_compute_mapgrid_batch): wait for the side stream, then redo any grid whose frontier queue
-		// overflowed with the scan-based kernel; h_seeds[0] = [status per (scene, grid)][seed offsets][seeds]
-		const int n_scenes = ctx->batch_wf_pending;
-		ctx->batch_wf_pending = 0;
-		CU(cudaEventSynchronize(ctx->wf_done[0]));
-		const size_t items = (size_t)n_scenes * HMP_NUM_MAPGRIDS;
-		const size_t n = (size_t)ctx->size_x * ctx->size_y;
-		const int* hs = (const int*)ctx->h_seeds[0].p;
-		const int* off = hs + items;
-		const int* d = (const int*)ctx->d_seeds[0].p;
-		bool any = false;
-		for (size_t it = 0; it < items; ++it) {
-			if (!hs[it]) continue;
-			const int s = (int)(it / HMP_NUM_MAPGRIDS);
-			CU(hmp_dev_launch_wavefront((const uint8_t*)ctx->d_costmaps.p + (size_t)s * ctx->costmap_stride, ctx->size_x, ctx->size_y,
-			                            d + items + (items + 1) + off[it], off[it + 1] - off[it], (float*)ctx->d_mapgrids.p + it * n, ctx->stream));
-			ctx->launches++;
-			any = true;
-		}
-		if (any) CU(cudaStreamSynchronize(ctx->stream));
-	}
-	// join the side streams of the pending wave fronts, then read their overflow flags with ONE synchronisation
-	int status[HMP_NUM_MAPGRIDS] = {0, 0, 0, 0};
-	bool any = false;
-	for (int g = 0; g < HMP_NUM_MAPGRIDS; ++g) {
-		if (!ctx->wavefront_pending[g]) continue;
-		CU(cudaStreamWaitEvent(ctx->stream, ctx->wf_done[g], 0));
-		CU(cudaMemcpyAsync(&status[g], ctx->d_seeds[g].p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-		any = true;
-	}
-	if (!any) return HMP_OK;
-	CU(cudaStreamSynchronize(ctx->stream));
-	for (int g = 0; g < HMP_NUM_MAPGRIDS; ++g) {
-		if (!ctx->wavefront_pending[g]) continue;
-		ctx->wavefront_pending[g] = false;
-		if (status[g]) {   // frontier queue overflowed: redo this grid with the scan-based kernel
-			const size_t n = (size_t)ctx->size_x * ctx->size_y;
-			CU(hmp_dev_launch_wavefront((const uint8_t*)ctx->d_costmaps.p, ctx->size_x, ctx->size_y, (const int*)ctx->d_seeds[g].p + 1,
-			                            ctx->n_seeds[g], (float*)ctx->d_mapgrids.p + (size_t)g * n, ctx->stream));
-			ctx->launches++;
-			CU(cudaStreamSynchronize(ctx->stream));
-		}
-	}
-	return HMP_OK;
-}
-
-// hmp_plan's form of the join: the plan stream waits for the side streams and copies the overflow flags into pinned memory;
-// the host does not wait here (it packs and uploads the world meanwhile, the wave fronts of a cycle take ~0.2 ms) and looks at
-// the flags after the cycle's final synchronisation (finish_wavefront_join). joined = number of pending grids.
-static int join_wavefronts_async(HmpContext* ctx, int* joined) {
-	*joined = 0;
-	int rc = ctx->h_small.ensure(64);
-	if (rc) return rc;
-	int32_t* hw = (int32_t*)ctx->h_small.p;
-	for (int g = 0; g < HMP_NUM_MAPGRIDS; ++g) {
-		hw[g] = 0;
-		if (!ctx->wavefront_pending[g]) continue;
-		CU(cudaStreamWaitEvent(ctx->stream, ctx->wf_done[g], 0));
-		CU(cudaMemcpyAsync(&hw[g], ctx->d_seeds[g].p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-		(*joined)++;
-	}
-	return HMP_OK;
-}
-// After the stream has been synchronised: a grid whose frontier queue overflowed (never observed for 200 x 200 windows) is
-// recomputed with the scan kernel; redo = 1 tells the caller that the cycle it just ran read an incomplete grid.
-static int finish_wavefront_join(HmpContext* ctx, int* redo) {
-	*redo = 0;
-	const int32_t* hw = (const int32_t*)ctx->h_small.p;
-	for (int g = 0; g < HMP_NUM_MAPGRIDS; ++g) {
-		if (!ctx->wavefront_pending[g]) continue;
-		ctx->wavefront_pending[g] = false;
-		if (hw[g]) {
-			const size_t n = (size_t)ctx->size_x * ctx->size_y;
-			CU(hmp_dev_launch_wavefront((const uint8_t*)ctx->d_costmaps.p, ctx->size_x, ctx->size_y, (const int*)ctx->d_seeds[g].p + 1,
-			                            ctx->n_seeds[g], (float*)ctx->d_mapgrids.p + (size_t)g * n, ctx->stream));
-			ctx->launches++;
-			*redo = 1;
-		}
-	}
-	if (*redo) CU(cudaStreamSynchronize(ctx->stream));
 	return HMP_OK;
 }
 
@@ -1130,15 +1038,11 @@ int hmp_compute_mapgrid(HmpContext* ctx, int32_t grid, const double* plan_xy, in
 		return HMP_E_NOT_READY;
 	}
 	CU(cudaSetDevice(ctx->device));
-	if (ctx->batch_wf_pending) {   // shares slot 0's staging buffers and side stream
-		int rcw = resolve_wavefronts(ctx);
-		if (rcw) return rcw;
-	}
 	const int sx = ctx->size_x, sy = ctx->size_y;
 	const size_t n = (size_t)sx * sy;
-	if (hmp_dev_wavefront_smem(sx, sy, 1) > ctx->max_smem_optin) {   // mark bits + both frontier queues
+	if (hmp_dev_wavefront_smem(sx, sy) > ctx->max_smem_optin) {
 		set_err("costmap too large for the on-device wave front (%zu bytes of shared memory needed, %zu available)",
-		        hmp_dev_wavefront_smem(sx, sy, 1), ctx->max_smem_optin);
+		        hmp_dev_wavefront_smem(sx, sy), ctx->max_smem_optin);
 		return HMP_E_CAPACITY;
 	}
 	// the costmap cells are needed for the NO_INFORMATION test of the seeds: keep a host copy from hmp_set_costmap
@@ -1148,33 +1052,37 @@ int hmp_compute_mapgrid(HmpContext* ctx, int32_t grid, const double* plan_xy, in
 	}
 	std::vector<int> seeds;
 	collect_seeds(ctx, ctx->h_cells.data(), plan_xy, n_plan, local_goal, seeds);
-	// per-slot staging so that the four grids of a cycle queue on the stream without a host synchronisation:
-	// [0] overflow status, [1..] seed cells
-	const size_t need = (1 + std::max<size_t>(1, seeds.size())) * sizeof(int);
+	// per-slot staging so that the four grids of a cycle queue on the stream without a host synchronisation, laid out like a
+	// batch of one: [0] [1] seed offsets, [2..] seed cells
+	const size_t need = (2 + std::max<size_t>(1, seeds.size())) * sizeof(int);
 	int rc = ctx->d_seeds[grid].ensure(need);
 	if (rc) return rc;
+	// the previous upload from this staging buffer (slot 0: possibly a batch's) has been consumed
+	if (ctx->seeds_event_valid[grid]) CU(cudaEventSynchronize(ctx->seeds_event[grid]));
 	if (need > ctx->h_seeds[grid].cap) {
 		CU(cudaStreamSynchronize(ctx->stream));
 		if ((rc = ctx->h_seeds[grid].ensure(need * 2))) return rc;
-	} else if (ctx->seeds_event_valid[grid]) {
-		CU(cudaEventSynchronize(ctx->seeds_event[grid]));   // previous upload from this staging buffer has been consumed
 	}
 	int* hs = (int*)ctx->h_seeds[grid].p;
 	hs[0] = 0;
-	if (!seeds.empty()) std::memcpy(hs + 1, seeds.data(), seeds.size() * sizeof(int));
+	hs[1] = (int)seeds.size();
+	if (!seeds.empty()) std::memcpy(hs + 2, seeds.data(), seeds.size() * sizeof(int));
 	// each grid has its own stream: hmp_set_costmap has synchronised (the cells are on the device), the previous plan has
 	// synchronised (nobody reads the MapGrid buffer), so the four single-block wave fronts of a cycle can overlap
 	cudaStream_t st = ctx->wf_stream[grid];
+	if (ctx->wf_after_batch[grid]) {   // a batch of wave fronts may still be writing this slot
+		CU(cudaStreamWaitEvent(st, ctx->wf_done[grid], 0));
+		ctx->wf_after_batch[grid] = false;
+	}
 	int* dsd = (int*)ctx->d_seeds[grid].p;
 	CU(cudaMemcpyAsync(dsd, hs, need, cudaMemcpyHostToDevice, st));
 	CU(cudaEventRecord(ctx->seeds_event[grid], st));
 	ctx->seeds_event_valid[grid] = true;
 	float* out = (float*)ctx->d_mapgrids.p + (size_t)grid * n;
-	CU(hmp_dev_launch_wavefront_queue((const uint8_t*)ctx->d_costmaps.p, sx, sy, dsd + 1, (int)seeds.size(), out, dsd, st));
+	CU(hmp_dev_launch_wavefront((const uint8_t*)ctx->d_costmaps.p, ctx->costmap_stride, sx, sy, dsd + 2, dsd, out, 1, 1, st));
 	CU(cudaEventRecord(ctx->wf_done[grid], st));
 	ctx->launches++;
 	ctx->wavefront_pending[grid] = true;
-	ctx->n_seeds[grid] = (int)seeds.size();   // overflow status is checked (and the scan kernel re-run) before the next plan
 	ctx->have_grid[grid] = true;
 	ctx->batch_grid_scenes = 0;
 	ctx->hv_prev[grid] = highest_valid_cost_prev;
@@ -1189,7 +1097,7 @@ int hmp_get_mapgrid(HmpContext* ctx, int32_t grid, double* target_dist_out) {
 	}
 	CU(cudaSetDevice(ctx->device));
 	{
-		int rc = resolve_wavefronts(ctx);
+		int rc = join_wavefronts(ctx);
 		if (rc) return rc;
 	}
 	const size_t n = (size_t)ctx->size_x * ctx->size_y;
@@ -1498,10 +1406,10 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 		// before the hv pass and the result copies are even queued); picked up after the final synchronisation
 		if ((rc = ctx->h_small.ensure(64))) return rc;
 		int32_t* hw = (int32_t*)ctx->h_small.p;
-		hw[4] = hw[5] = hw[6] = 0;
-		CU(cudaMemcpyAsync(&hw[4], r_count_dev[0], sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-		CU(cudaMemcpyAsync(&hw[6], r_count_dev[0] + NS, sizeof(int32_t), cudaMemcpyDeviceToHost, st));   // r_unrel of scene 0
-		if (r_count_dev[1]) CU(cudaMemcpyAsync(&hw[5], r_count_dev[1], sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+		hw[0] = hw[1] = hw[2] = 0;
+		CU(cudaMemcpyAsync(&hw[0], r_count_dev[0], sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+		CU(cudaMemcpyAsync(&hw[2], r_count_dev[0] + NS, sizeof(int32_t), cudaMemcpyDeviceToHost, st));   // r_unrel of scene 0
+		if (r_count_dev[1]) CU(cudaMemcpyAsync(&hw[1], r_count_dev[1], sizeof(int32_t), cudaMemcpyDeviceToHost, st));
 	}
 	// highest_valid_cost_ of the MapGrid critics as the reference's sequential, early-exiting loop would leave it: needs the final
 	// explored totals (refined leaders included) for the best-so-far every candidate was scored against
@@ -1524,9 +1432,9 @@ static int run_cycle(HmpContext* ctx, const DevParams& D, const std::vector<doub
 	};
 	if ((rc = read_back())) return rc;
 	if (ctx->precise == 2) {
-		ctx->last_n_leaders = ((const int32_t*)ctx->h_small.p)[4];
-		ctx->last_n_leaders2 = ((const int32_t*)ctx->h_small.p)[5];
-		ctx->last_unreliable = ((const int32_t*)ctx->h_small.p)[6];
+		ctx->last_n_leaders = ((const int32_t*)ctx->h_small.p)[0];
+		ctx->last_n_leaders2 = ((const int32_t*)ctx->h_small.p)[1];
+		ctx->last_unreliable = ((const int32_t*)ctx->h_small.p)[2];
 	} else {
 		ctx->last_unreliable = 0;
 	}
@@ -1660,7 +1568,6 @@ int hmp_plan(HmpContext* ctx, const HmpWorld* world, const HmpSampling* sampling
 		return HMP_E_NOT_READY;
 	}
 	CU(cudaSetDevice(ctx->device));
-	if (ctx->batch_wf_pending && (rc = resolve_wavefronts(ctx))) return rc;
 	int T = compute_steps(ctx->params.general, std::hypot(world->vel_x, world->vel_y), world->vel_th);
 	if (T < 1 || T > HMP_MAX_STEPS) {
 		set_err("rollout has %d steps, supported 1..%d", T, HMP_MAX_STEPS);
@@ -1684,17 +1591,11 @@ int hmp_plan(HmpContext* ctx, const HmpWorld* world, const HmpSampling* sampling
 	pack_scene(ctx, *world, ctx->hv_prev, D.dt_d, (unsigned char*)ctx->h_stage.p, D.n_equi);
 	uint32_t used = reinterpret_cast<DevScene*>(ctx->h_stage.p)->blob_bytes;
 	// device wave fronts of this cycle (hmp_compute_mapgrid) have been running on their side streams while the host packed the
-	// world; the plan stream joins them here, their overflow flags are read with the cycle's final synchronisation
-	int joined = 0;
-	if ((rc = join_wavefronts_async(ctx, &joined))) return rc;
+	// world; the plan stream joins them here
+	if ((rc = join_wavefronts(ctx))) return rc;
 	CU(cudaMemcpyAsync(ctx->d_scenes.p, ctx->h_stage.p, used, cudaMemcpyHostToDevice, ctx->stream));
 	PlanLaunch pl{1, used, n_extra, T};
 	if ((rc = run_cycle(ctx, D, amp_table, extra, n_extra, equi, pl, result, poses_out, poses_capacity))) return rc;
-	if (joined) {
-		int redo = 0;
-		if ((rc = finish_wavefront_join(ctx, &redo))) return rc;
-		if (redo && (rc = run_cycle(ctx, D, amp_table, extra, n_extra, equi, pl, result, poses_out, poses_capacity))) return rc;
-	}
 	// Escalation (hmp_set_escalation): the refinement has just compared the FP32 and FP64 totals of the leaders. When many of them
 	// disagree by more than 1 % the FP32 ranking of THIS plan is unreliable (chaotic rollouts around a spinning robot: the true
 	// winner can sit thousands of ranks down, DESIGN 4b) -- the plan is redone as an exact FP64 sweep on the resident inputs.
@@ -1730,7 +1631,7 @@ static int upload_batch_costmaps(HmpContext* ctx, const uint8_t* cells, int n_sc
 }
 
 // MapGridCostFunction::setTargetPoses + prepare() for n_scenes x 4 grids in ONE launch: seeds on the host, the wave fronts on
-// the device (one block per grid, mapgrid_wavefront_batch_kernel), so that a batch uploads 1 byte per cell (the costmap)
+// the device (one block per grid, hmp_dev_launch_wavefront), so that a batch uploads 1 byte per cell (the costmap)
 // instead of 17 (costmap + four float grids).
 int hmp_compute_mapgrid_batch(HmpContext* ctx, int32_t n_scenes, const uint8_t* cells, const double* const plan_xy[HMP_NUM_MAPGRIDS],
                               const int32_t* const plan_start[HMP_NUM_MAPGRIDS], const int32_t local_goal[HMP_NUM_MAPGRIDS]) {
@@ -1752,10 +1653,10 @@ int hmp_compute_mapgrid_batch(HmpContext* ctx, int32_t n_scenes, const uint8_t* 
 			}
 	}
 	CU(cudaSetDevice(ctx->device));
-	if ((rc = resolve_wavefronts(ctx))) return rc;
+	if ((rc = join_wavefronts(ctx))) return rc;
 	const int sx = ctx->size_x, sy = ctx->size_y;
 	const size_t n = (size_t)sx * sy;
-	if (hmp_dev_wavefront_smem(sx, sy, 1) > ctx->max_smem_optin) {
+	if (hmp_dev_wavefront_smem(sx, sy) > ctx->max_smem_optin) {
 		set_err("costmap too large for the on-device wave front");
 		return HMP_E_CAPACITY;
 	}
@@ -1765,7 +1666,7 @@ int hmp_compute_mapgrid_batch(HmpContext* ctx, int32_t n_scenes, const uint8_t* 
 		set_err("hmp_compute_mapgrid_batch needs the per-scene costmap cells (%d scenes resident, %d asked)", ctx->costmap_scenes, n_scenes);
 		return HMP_E_NOT_READY;
 	}
-	// seeds of all (scene, grid) pairs on the host threads: [status n_items][offsets n_items + 1][seeds ...]
+	// seeds of all (scene, grid) pairs on the host threads: [offsets n_items + 1][seeds ...]
 	const size_t items = (size_t)n_scenes * HMP_NUM_MAPGRIDS;
 	std::vector<std::vector<int>> seeds(items);
 	std::vector<uint8_t> cells_dev;   // only when the cells are not passed again (seed test needs them): read back
@@ -1791,13 +1692,11 @@ int hmp_compute_mapgrid_batch(HmpContext* ctx, int32_t n_scenes, const uint8_t* 
 	}
 	size_t total = 0;
 	for (auto& v : seeds) total += v.size();
-	const size_t words = items + (items + 1) + std::max<size_t>(1, total);
+	const size_t words = (items + 1) + std::max<size_t>(1, total);
 	if ((rc = ctx->d_seeds[0].ensure(words * sizeof(int)))) return rc;
 	CU(cudaStreamSynchronize(ctx->stream));
 	if ((rc = ctx->h_seeds[0].ensure(words * sizeof(int)))) return rc;
-	int* hs = (int*)ctx->h_seeds[0].p;
-	std::memset(hs, 0, items * sizeof(int));
-	int* off = hs + items;
+	int* off = (int*)ctx->h_seeds[0].p;
 	int* sd = off + items + 1;
 	size_t pos = 0;
 	for (size_t it = 0; it < items; ++it) {
@@ -1807,18 +1706,22 @@ int hmp_compute_mapgrid_batch(HmpContext* ctx, int32_t n_scenes, const uint8_t* 
 	}
 	off[items] = (int)pos;
 	if ((rc = ctx->d_mapgrids.ensure(n * HMP_NUM_MAPGRIDS * sizeof(float) * n_scenes))) return rc;
-	// The wave fronts run on a side stream and are NOT waited for here: the caller's next step (hmp_plan_batch packs and uploads
-	// the worlds) overlaps them; resolve_wavefronts() joins the stream and checks the overflow flags before the first kernel
-	// that reads the grids. The costmaps are on the device already (upload_batch_costmaps synchronised).
+	// The wave fronts run on slot 0's side stream and are NOT waited for here: the caller's next step (hmp_plan_batch packs and
+	// uploads the worlds) overlaps them; join_wavefronts() orders them before the first kernel that reads the grids. The
+	// costmaps are on the device already (upload_batch_costmaps synchronised).
 	cudaStream_t st = ctx->wf_stream[0];
 	int* d = (int*)ctx->d_seeds[0].p;
-	CU(cudaMemcpyAsync(d, hs, words * sizeof(int), cudaMemcpyHostToDevice, st));
-	CU(hmp_dev_launch_wavefront_batch((const uint8_t*)ctx->d_costmaps.p, ctx->costmap_stride, sx, sy, d + items + (items + 1), d + items,
-	                                  (float*)ctx->d_mapgrids.p, d, n_scenes, st));
+	CU(cudaMemcpyAsync(d, off, words * sizeof(int), cudaMemcpyHostToDevice, st));
+	CU(cudaEventRecord(ctx->seeds_event[0], st));   // slot 0's staging buffer: hmp_compute_mapgrid(0) waits for this copy
+	ctx->seeds_event_valid[0] = true;
+	CU(hmp_dev_launch_wavefront((const uint8_t*)ctx->d_costmaps.p, ctx->costmap_stride, sx, sy, d + items + 1, d, (float*)ctx->d_mapgrids.p,
+	                            HMP_NUM_MAPGRIDS, n_scenes, st));
 	ctx->launches++;
-	CU(cudaMemcpyAsync(hs, d, items * sizeof(int), cudaMemcpyDeviceToHost, st));   // status words back into the pinned staging buffer
-	CU(cudaEventRecord(ctx->wf_done[0], st));
-	ctx->batch_wf_pending = n_scenes;
+	for (int g = 0; g < HMP_NUM_MAPGRIDS; ++g) {   // the batch writes every slot of scene 0
+		CU(cudaEventRecord(ctx->wf_done[g], st));
+		ctx->wf_after_batch[g] = true;
+	}
+	ctx->wavefront_pending[0] = true;
 	for (bool& b : ctx->have_grid) b = true;
 	ctx->batch_grid_scenes = n_scenes;
 	ctx->last_valid = false;
@@ -1836,7 +1739,7 @@ int hmp_set_mapgrids_batch_f32(HmpContext* ctx, int32_t n_scenes, const float* c
 		return HMP_E_INVALID;
 	}
 	CU(cudaSetDevice(ctx->device));
-	if ((rc = resolve_wavefronts(ctx))) return rc;
+	if ((rc = join_wavefronts(ctx))) return rc;
 	const size_t n = (size_t)ctx->size_x * ctx->size_y;
 	if ((rc = ctx->d_mapgrids.ensure(n * HMP_NUM_MAPGRIDS * sizeof(float) * n_scenes))) return rc;
 	for (int g = 0; g < HMP_NUM_MAPGRIDS; ++g)   // [scene][grid][cells] on the device, [scene][cells] per grid on the host
@@ -1960,7 +1863,7 @@ int hmp_plan_batch(HmpContext* ctx, const HmpWorld* worlds, int32_t n_scenes, co
 	CU(cudaMemcpyAsync(ctx->d_scenes.p, hs, stride * n_scenes, cudaMemcpyHostToDevice, ctx->stream));
 	CU(cudaStreamSynchronize(ctx->stream));
 	// device wave fronts still in flight (hmp_compute_mapgrid[_batch]) ran beside the packing above; join them now
-	if ((rc = resolve_wavefronts(ctx))) return rc;
+	if ((rc = join_wavefronts(ctx))) return rc;
 	if (cells) {
 		if ((rc = upload_batch_costmaps(ctx, cells, n_scenes))) return rc;
 	}
@@ -2231,7 +2134,7 @@ int hmp_compute_cost_cloud(HmpContext* ctx, float* cloud6, uint8_t* valid) {
 		}
 	}
 	CU(cudaSetDevice(ctx->device));
-	if ((rc = resolve_wavefronts(ctx))) return rc;
+	if ((rc = join_wavefronts(ctx))) return rc;
 	DevParams D;
 	if ((rc = debug_params(ctx, D))) return rc;
 	const size_t n = (size_t)ctx->size_x * ctx->size_y;
